@@ -3,6 +3,7 @@
 the reference.  Contract: one JSON line on stdout (rank 0).
 
   python bench.py --gpus 1 --steps 5 --warmup 3            # our arm
+  python bench.py --gpus 1 --steps 5 --warmup 3 --dump-outputs DIR   # ... and the last timed step's outputs as DIR/*.npy
   python bench.py --impl reference --steps 2 --warmup 1    # the reference's algorithms on the host cores (oracle port)
   python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
@@ -96,6 +97,14 @@ class ClockSampler:
                 "reasons": sorted(reasons), "samples": len(sm)}
 
 
+DUMP_NTT_ROWS = 1 << 16    # --dump-outputs: rows of an NTT output kept (a fixed, seeded sample; 4 MB per transform)
+
+
+def u64_as_f64(limbs: np.ndarray) -> np.ndarray:
+    """u64 limbs -> their 32-bit halves (low half first) as float64, which holds every such value exactly"""
+    return np.ascontiguousarray(limbs, dtype=np.uint64).view(np.uint32).astype(np.float64)
+
+
 def msm_work(n: int, c: int, W: int, limbs32: int):
     """SURVEY.md §8(d): Fq modmuls = 10*n*W + 14*2^c*W ; wide MADs per modmul = 2L^2 + L ; bytes = n*(2*8N + 32)"""
     modmuls = 10.0 * n * W + 14.0 * (1 << c) * W
@@ -155,7 +164,7 @@ def run_reference(args):
     x[:, 3] &= np.uint64((1 << 62) - 1)
     C.fft(1, x[: 1 << 16], False, None, threads)
     tn = []
-    for _ in range(max(1, min(args.steps, 3))):
+    for _ in range(args.steps):
         t0 = time.perf_counter()
         C.lib().ark_fft(1, x.ctypes.data_as(ctypes.POINTER(ctypes.c_uint64)), args.log_n_ntt, 0, None, threads)
         tn.append(time.perf_counter() - t0)
@@ -167,10 +176,11 @@ def run_reference(args):
         "steps": args.steps, "warmup": args.warmup, "ms_per_step": t_full * 1e3, "higher_is_better": True, "scaling": "strong",
         "vs_baseline": None, "dtype": "u64 limbs (Montgomery, 6x64-bit Fq / 4x64-bit Fr)", "data": "synthetic",
         "config": {"workload": "BLS12-381 G1 VariableBaseMSM n=2^%d, uniform scalars" % log_n, "seed": args.seed},
-        "cpu_baseline": {"value": v, "unit": "MSM/s", "cores": threads, "kind": "port", "sample": sample},
+        "cpu_baseline": {"value": v, "unit": "MSM/s", "cores": threads, "kind": "port", "sample": sample, "steps": args.steps,
+                         "warmup": args.warmup},
         "e2e": {"value": v, "unit": "MSM/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "ntt": {"metric": "BLS12-381 Fr NTT/s @2^%d" % args.log_n_ntt, "value": 1.0 / statistics.mean(tn), "unit": "NTT/s",
-                "ms_per_step": statistics.mean(tn) * 1e3},
+                "ms_per_step": statistics.mean(tn) * 1e3, "steps": len(tn)},
         "gpu_launches": 0,
     }
     print(json.dumps(line), flush=True)
@@ -180,7 +190,9 @@ def run_reference(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5,
+                    help="timed steps of every leg of the arm; the b200 arm's cpu_baseline is one step of the reference arm (its own "
+                         "steps/warmup are reported in it), a bounded sample: at 2^26 that step alone takes about a minute")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--log-n-msm", type=int, default=26)
@@ -196,7 +208,15 @@ def main():
     ap.add_argument("--no-verify", action="store_true")
     ap.add_argument("--no-ntt", action="store_true", help="skip the NTT leg (MSM tuning runs)")
     ap.add_argument("--ref-full", action="store_true", help="--impl reference: time the full n instead of the n/4 sample")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="--impl b200: write what the last timed step of the device-resident legs returned as DIR/<name>.npy (float64, "
+                         "exact 32-bit halves of the u64 limbs): msm_affine (the MSM `value` leg), ntt_fft and ntt_ifft (%d seeded rows "
+                         "of each transform); the host-buffer e2e legs compute the same MSM, checked by e2e.same_result" % DUMP_NTT_ROWS)
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -293,6 +313,18 @@ def main():
         phase[k] /= args.steps
     clocks = clk.summary()
 
+    dump = {}     # --dump-outputs: name -> float64 array, written by rank 0 once the legs are done
+
+    def write_dump():
+        if rank == 0 and args.dump_outputs:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in dump.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
+
+    if args.dump_outputs:
+        # the affine point is the group element itself; the Jacobian limbs the call returns depend on the order of the additions
+        dump["msm_affine"] = u64_as_f64(ab.into_affine(cv, res))
+
     # ---------------- verification: MSM(b_i*G, s_i) == (sum s_i*b_i mod r) * G, all ranks' shards included
     verified = None
     if not args.no_verify:
@@ -340,7 +372,7 @@ def main():
             dt = time.perf_counter() - t0
             barrier()
             return max_over_ranks(dt) / steps, r
-        e2e_steps = max(1, min(args.steps, 3))
+        e2e_steps = args.steps
         h_bases = torch.empty((n_chunk, 2 * N), dtype=torch.int64).pin_memory()
         h_scal = torch.empty((n_chunk, 4), dtype=torch.int64).pin_memory()
         h_bases.copy_(d_bases[c_lo:c_lo + n_chunk])
@@ -365,6 +397,7 @@ def main():
             print(json.dumps({"metric": "msm-only tuning run", "value": 1000.0 / ms_msm, "unit": "MSM/s", "ms_per_step": ms_msm,
                               "phases_ms": phase, "window_c": tm["c"], "windows": tm["windows"], "verified": verified,
                               "e2e": e2e, "clocks": clocks, "gpu_launches": launches}), flush=True)
+        write_dump()
         if world > 1:
             dist.destroy_process_group()
         return
@@ -378,9 +411,15 @@ def main():
     ntt_l0 = L.b200_launch_count()
     ms_ntt, _ = timed(lambda: dom.fft_in_place(d_x), args.steps)
     ntt_launches = int(L.b200_launch_count() - ntt_l0)
+    if args.dump_outputs:
+        rows = np.random.default_rng(args.seed).choice(n_ntt, size=min(n_ntt, DUMP_NTT_ROWS), replace=False)
+        rows = torch.from_numpy(np.sort(rows)).to(dev)
+        dump["ntt_fft"] = u64_as_f64(d_x[rows].cpu().numpy().view(np.uint64))
     for _ in range(args.warmup):   # also builds the inverse plan outside the timed region
         dom.ifft_in_place(d_x)
     ms_intt, _ = timed(lambda: dom.ifft_in_place(d_x), args.steps)
+    if args.dump_outputs:
+        dump["ntt_ifft"] = u64_as_f64(d_x[rows].cpu().numpy().view(np.uint64))
     # round trip property on the timed data: (warmup + steps) forward then as many inverse transforms restore x0
     ntt_ok = bool(torch.equal(d_x, x0))
     ntt_e2e = None
@@ -390,9 +429,9 @@ def main():
         hxn = hx.numpy().view(np.uint64)
         dom.fft_in_place(hxn)
         t0 = time.perf_counter()
-        for _ in range(max(1, min(args.steps, 3))):
+        for _ in range(args.steps):
             dom.fft_in_place(hxn)
-        dt = (time.perf_counter() - t0) / max(1, min(args.steps, 3))
+        dt = (time.perf_counter() - t0) / args.steps
         ntt_e2e = {"value": world / max_over_ranks(dt), "unit": "NTT/s", "h2d_bytes_per_step": n_ntt * 32 * world,
                    "d2h_bytes_per_step": n_ntt * 32 * world}
 
@@ -467,6 +506,7 @@ def main():
                                       "frac": 136.0 * (n_ntt / 2 * args.log_n_ntt) / (ms_ntt * 1e-3) / IMAD_PEAK_WIDE_PER_S}},
         }
         print(json.dumps(line), flush=True)
+    write_dump()
     if world > 1:
         dist.destroy_process_group()
 
